@@ -8,6 +8,7 @@ N > 1 the single NCCL all-reduce of that buffer.  Workload = BASELINE.json confi
 (OTTER-Image-MPT7B shape, per-GPU batch 8, 1 image/sample, L = 256, bf16), weak scaling over ranks.
 
   python bench.py [--gpus N --steps K --warmup W]            this repo's CUDA path (one rank per GPU)
+  python bench.py --dump-outputs DIR [...]                    also writes the last timed step's loss and gradients
   python bench.py --impl reference [...]                      the reference's CPU implementation of the same path
 
 Numerics of every GPU number printed here: production mode = bf16 operands, fp32 accumulation / softmax / LayerNorm
@@ -32,6 +33,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 import torch  # noqa: E402
 
@@ -168,6 +170,7 @@ class HotPath:
         self.loss_host = torch.zeros(1).pin_memory()
         self.graphed = None
         self.hidden = None
+        self.loss = None
         self.launches_per_step = None
         self.prefetch = None
 
@@ -226,6 +229,7 @@ class HotPath:
         import torch.distributed as dist
         loss = self.graphed[1].replay() if self.graphed is not None else \
             self.train_step(self.hidden, self.d_hid, self.d_loc)
+        self.loss = loss
         work = self.flat.all_reduce(async_op=True)
         self.run_clip()
         if work is not None:
@@ -492,6 +496,32 @@ def self_check(hp):
             "oracle_seconds": round(time.perf_counter() - t0, 1)}
 
 
+DUMP_SAMPLE = 65536                 # gradient entries kept per parameter by --dump-outputs
+
+
+def dump_outputs(hp, out_dir):
+    """What the last step handed its caller, the loss and the fp32 gradient of every trainable parameter, as
+    <out_dir>/<name>.npy in float32.  A gradient with more than DUMP_SAMPLE entries is sampled at positions drawn from a
+    generator seeded with the parameter's name, so that two builds of the project can be compared entry for entry."""
+    import zlib
+
+    import numpy as np
+    torch.cuda.synchronize()
+    arrays = {"loss": hp.loss}
+    for prefix, mod in (("perceiver", hp.perceiver), ("gated", hp.gated)):
+        for pname, p in mod.named_parameters():
+            name = f"grad.{prefix}.{pname}"
+            g = p.grad.detach().reshape(-1)
+            if g.numel() > DUMP_SAMPLE:
+                gen = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+                g = g[torch.randint(g.numel(), (DUMP_SAMPLE,), generator=gen).sort().values.to(g.device)]
+            arrays[name] = g
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    return len(arrays), sum(t.numel() * 4 for t in arrays.values())
+
+
 def fuyu_patch_linear_times(dev):
     """BASELINE configs[4] (OtterHD/Fuyu patch-linear, no vision encoder): Linear(2700 -> 4096, bias) on N_p patches +
     scatter into the word embeddings, through otter_b200.modeling_fuyu (reference signature)."""
@@ -749,6 +779,9 @@ def run_cuda(args):
     launches = hp.launches_per_step
     clocks = sampler.stop() if sampler else None
     ms_e2e = hp.timed(args.steps, e2e=True)
+    if args.dump_outputs and rank == 0:
+        n, nbytes = dump_outputs(hp, args.dump_outputs)
+        log(f"last step's loss and gradients: {n} arrays, {nbytes / 2 ** 20:.1f} MiB in {args.dump_outputs}")
 
     peaks = {}
     try:
@@ -1075,7 +1108,12 @@ def main():
     ap.add_argument("--ref-batch", type=int, default=0, help="reference arm: batch per step (default: --per-gpu-batch)")
     ap.add_argument("--ref-budget-s", type=float, default=150.0, help="reference arm: wall-clock bound of the timed steps")
     ap.add_argument("--ref-port", action="store_true", help="reference arm: time oracle/restatement.py instead")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and (sampled) parameter gradients to "
+                         "DIR/<name>.npy, to compare the outputs of two builds on identical inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "otter_b200":
+        ap.error("--dump-outputs writes what the CUDA arm computed; it does not apply to --impl reference")
     BASE_CFG["L"] = args.seq_len
     if args.impl == "reference":
         run_reference(args)

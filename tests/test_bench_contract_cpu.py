@@ -77,3 +77,44 @@ def test_allreduce_alone_record(monkeypatch):
     assert _Flat.calls == 12                                    # 2 warm-up + 10 timed
     assert r["ms"] == 5.0 and r["wire_bytes"] == 2_000_000_000 and r["iters"] == 10
     assert abs(r["busbw_gbs"] - 2 * 7 / 8 * 2e9 / 5e-3 / 1e9) < 0.1      # 700 GB/s
+
+
+def test_dump_outputs_files(tmp_path, monkeypatch):
+    """--dump-outputs: one float32 .npy per array (the loss, every trainable parameter's gradient), large gradients
+    sampled at the same positions on every run, and at the timed workload's parameter shapes under the 64 MB bound."""
+    import types
+
+    import numpy as np
+    import torch
+    import bench
+    from otter_b200.modeling_otter import OtterGatedCrossAttentionBlock, OtterPerceiverResampler
+
+    monkeypatch.setattr(torch.cuda, "synchronize", lambda *a, **k: None)
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    torch.manual_seed(0)
+    hp = types.SimpleNamespace(loss=torch.tensor([0.25]), perceiver=OtterPerceiverResampler(dim=32, depth=1),
+                               gated=torch.nn.ModuleList([OtterGatedCrossAttentionBlock(dim=64, dim_visual=32)]))
+    params = [(f"grad.{pre}.{n}", p) for pre, m in (("perceiver", hp.perceiver), ("gated", hp.gated))
+              for n, p in m.named_parameters()]
+    for _, p in params:
+        p.grad = torch.randn_like(p)
+    n, nbytes = bench.dump_outputs(hp, str(tmp_path / "a"))
+    bench.dump_outputs(hp, str(tmp_path / "b"))
+    names = sorted(f[:-4] for f in os.listdir(tmp_path / "a"))
+    assert n == len(names) == len(params) + 1 and names == sorted(["loss"] + [k for k, _ in params])
+    assert np.array_equal(np.load(tmp_path / "a" / "loss.npy"), hp.loss.numpy())
+    total = 4
+    for name, p in params:
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, b) and a.size == min(p.numel(), 1000)
+        g = p.grad.reshape(-1).numpy()
+        assert np.array_equal(a, g) if p.numel() <= 1000 else np.isin(a, g).all()
+        total += a.nbytes
+    assert any(p.numel() > 1000 for _, p in params) and nbytes == total
+    monkeypatch.undo()
+    with torch.device("meta"):                                  # the timed workload's modules, shapes only
+        per = OtterPerceiverResampler(dim=bench.BASE_CFG["vis_dim"])
+        gated = [OtterGatedCrossAttentionBlock(dim=bench.BASE_CFG["D"], dim_visual=bench.BASE_CFG["vis_dim"])
+                 for _ in range(bench.BASE_CFG["n_gated"])]
+    sizes = [p.numel() for m in [per] + gated for p in m.parameters()]
+    assert 4 * (1 + sum(min(s, bench.DUMP_SAMPLE) for s in sizes)) <= 64 * 2 ** 20

@@ -1,9 +1,9 @@
 """GPU: the drop-in boundary exercised the way the reference's own callers use it.
 
-  * the reference's `forward_pass` (pipeline/train/instruction_following.py:73-103), extracted VERBATIM by AST from the
-    reference file (from /root/reference here, from the archive oracle/build_ref.py packs on the GPU box) and called
-    on otter_b200's OtterForConditionalGeneration — the loss must equal the one the same function returned for the
-    reference model (fixture forward_pass_otter.pt);
+  * the reference's `forward_pass` (pipeline/train/instruction_following.py:73-103): the model call it makes for an Otter
+    model (recorded by oracle/make_golden_live.py in caller_functions.pt: which inputs reach which keyword, in which
+    dtype, which output element is the loss) replayed on otter_b200's OtterForConditionalGeneration — the loss must
+    equal the one the same function returned for the reference model (fixture forward_pass_otter.pt);
   * the OpenFlamingo twin classes (modeling_flamingo.py:87-985) under their own names, against a reference Flamingo
     golden and the reference's state-dict keys / trainable set;
   * OtterForConditionalGeneration over an MPT text config (class-name dispatch modeling_otter.py:500-509), with this
@@ -16,7 +16,6 @@ import types
 import pytest
 import torch
 
-from oracle import ref_shims
 from oracle.ref_shims import FakeTokenizer
 from oracle.seeded import load_seeded_, seeded_tensor
 
@@ -59,21 +58,20 @@ def _check(model, out, g, what, loss_tol=2e-2):
     check_grads(model.named_parameters(), g["grads"], what, norm_tol=5e-2, samp_tol=1e-1, gate_tol=0.12)
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason="needs /root/reference or oracle/_ref (build())")
 def test_reference_forward_pass_runs_on_the_drop_in(monkeypatch):
-    from oracle.make_golden_r2 import load_forward_pass
     from otter_b200 import otter_hf
     monkeypatch.setattr(otter_hf, "AutoTokenizer", FakeTokenizer)
-    forward_pass = load_forward_pass()                      # the reference's own function object
+    call = gold("caller_functions.pt")["forward_pass"]     # the call the reference's forward_pass makes
+    assert call["model_name"] == "otter" and call["autocast_type"] == "bfloat16"   # the training recipe's cast (:99)
     g = gold("forward_pass_otter.pt")
     model = otter_hf.OtterForConditionalGeneration(_llama_cfg(g, otter_hf.OtterConfig))
     load_seeded_(model, g["seed"], kinds=EMB_KINDS)
     model.to(DEV)
     vision_x = seeded_tensor("in.fp.vision_x", (2, 1, 1, 3, 224, 224), g["input_seed"], "randn").to(DEV)
     lang_x, labels = g["lang_x"].to(DEV), g["labels"].to(DEV)
-    args = types.SimpleNamespace(model_name="otter")
-    loss = forward_pass(args, model, model.text_tokenizer, vision_x, lang_x, torch.ones_like(lang_x), labels, DEV,
-                        torch.bfloat16, {})                 # autocast_type bf16: the training recipe's cast (:99)
+    inputs = {"images": vision_x, "input_ids": lang_x, "attention_mask": torch.ones_like(lang_x), "labels": labels}
+    out = model(**{k: inputs[a["from"]].to(getattr(torch, a["dtype"])) for k, a in call["kwargs"].items()})
+    loss = out[call["output_index"]]
     _check(model, types.SimpleNamespace(loss=loss), g, "forward_pass")
 
 

@@ -1,14 +1,14 @@
-"""CPU: the frozen-LM oracle (oracle/restatement_lm.py, SURVEY.md §8f rank 1) against the golden fixture generated from the
-unmodified reference MPTBlock, and — when /root/reference is present — against the live reference classes."""
+"""CPU: the frozen-LM oracle (oracle/restatement_lm.py, SURVEY.md §8f rank 1) against golden fixtures generated from the
+unmodified reference MPTBlock (oracle/make_golden_lm.py, oracle/make_golden_live.py)."""
 import os
 
-import pytest
 import torch
 
-from oracle import ref_shims
 from oracle import restatement_lm as R
+from oracle.seeded import seeded_state, seeded_tensor
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "mpt_block_tiny.pt")
+GOLD_LIVE = os.path.join(os.path.dirname(__file__), "golden", "mpt_block_live.pt")
 
 
 def test_alibi_slopes_power_of_two_and_not():
@@ -44,14 +44,11 @@ def test_causality_and_shift_property():
     assert not torch.allclose(y[:, S // 2:], y2[:, S // 2:])
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason="needs /root/reference (build container only)")
 def test_against_live_reference_block():
-    from oracle.make_golden_lm import reference_block
-    blk, run = reference_block(128, 8, no_bias=True, seed=5)
-    x = torch.randn(2, 40, 128, generator=torch.Generator().manual_seed(2))
-    want = run(x)
-    got = R.mpt_block(x, dict(blk.state_dict()), 8)
-    assert torch.allclose(got, want, rtol=1e-5, atol=1e-5)
-    blk_b, run_b = reference_block(64, 4, no_bias=False, seed=6)        # with biases (generic MPT configs)
-    xb = torch.randn(1, 9, 64, generator=torch.Generator().manual_seed(3))
-    assert torch.allclose(R.mpt_block(xb, dict(blk_b.state_dict()), 4), run_b(xb), rtol=1e-5, atol=1e-5)
+    """Head dim 16 without biases, and with biases (generic MPT configs), vs the reference block's outputs."""
+    gold = torch.load(GOLD_LIVE)
+    assert any(not c["no_bias"] for c in gold.values())
+    for name, c in gold.items():
+        x = seeded_tensor(f"in.live.mpt.{name}", c["x_shape"], c["seed"], "randn")
+        got = R.mpt_block(x, seeded_state(c["shapes"], c["seed"]), c["H"])
+        assert torch.allclose(got, c["y"], rtol=1e-5, atol=1e-5), name
