@@ -756,6 +756,15 @@ extern "C" int otb_gemm_bf16(const void* A, int a_mn_major, int64_t lda, const v
                              int M, int N, int K, const otb_gemm_epilogue* e, void* stream) {
   using namespace otb;
   OTB_CHECK_ARG(A && B && e && e->out, "otb_gemm_bf16: null pointer");
+  // Operands go through TMA and the epilogue reads / writes 16 B vectors (uint4 / float4): every matrix and the bias
+  // must start on a 16-byte boundary.  A misaligned pointer is an argument error, not a fault inside the kernel.
+  {
+    const void* ptrs[7] = {A, B, e->out, e->bias, e->residual, e->aux_in, e->aux_out};
+    const char* names[7] = {"A", "B", "out", "bias", "residual", "aux_in", "aux_out"};
+    for (int i = 0; i < 7; ++i)
+      OTB_CHECK_ARG((reinterpret_cast<uintptr_t>(ptrs[i]) & 15) == 0, "otb_gemm_bf16: %s is not 16-byte aligned",
+                    names[i]);
+  }
   OTB_CHECK_ARG(M > 0 && N > 0 && K > 0, "otb_gemm_bf16: bad shape %d %d %d", M, N, K);
   OTB_CHECK_ARG(N % 8 == 0, "otb_gemm_bf16: N=%d must be a multiple of 8", N);
   OTB_CHECK_ARG(e->ld_out % 8 == 0 && e->ld_out >= N, "otb_gemm_bf16: bad ld_out");
@@ -785,8 +794,7 @@ extern "C" int otb_gemm_bf16(const void* A, int a_mn_major, int64_t lda, const v
   // Outputs leave through the smem-staged TMA-store / reduce-add epilogue (r02: FFN up GELU+aux 194 -> 164 us, fp32
   // wgrad 206 -> 171 us, step +3 %; profiles/r02_gemm_selftest_bench.md).  OTB_GEMM_EPI_TMA=0 selects direct stores.
   static const bool epi_tma = [] { const char* v = getenv("OTB_GEMM_EPI_TMA"); return !(v && v[0] == '0'); }();
-  ep.tma_out = (epi_tma && !e->res_fp32 && (reinterpret_cast<uintptr_t>(e->out) & 15) == 0 &&
-                (!e->out_fp32 || e->ld_out % 4 == 0)) ? 1 : 0;
+  ep.tma_out = (epi_tma && !e->res_fp32 && (!e->out_fp32 || e->ld_out % 4 == 0)) ? 1 : 0;
   ep.cls = -1;
   if (ep.tma_out && e->res_fp32 == 0) {
     const bool scaled = (e->scale_ptr != nullptr) || e->alpha != 1.0f;

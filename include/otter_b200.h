@@ -50,7 +50,8 @@ int otb_abi_sizeof(int which);
  *   a_mn_major = 1 : A is stored [K][M] row-major (lda >= M)         (dY^T for wgrad, no transpose copy)
  *   b_mn_major = 0 : B is stored [N][K] row-major (ldb >= K)         (nn.Linear weight for forward)
  *   b_mn_major = 1 : B is stored [K][N] row-major (ldb >= N)         (weight for dgrad, X for wgrad)
- * Requirements: lda, ldb, ld_out, ld_aux, ld_res multiples of 8; pointers 16-byte aligned;
+ * Requirements: lda, ldb, ld_out, ld_aux, ld_res multiples of 8; A, B, out, bias, residual, aux_in and aux_out
+ *   16-byte aligned (otherwise OTB_ERR_INVALID naming the operand);
  *   N multiple of 8; for an MN-major operand its MN extent must be a multiple of 8.
  *
  * Epilogue (all optional, applied in this order on the fp32 accumulator v):

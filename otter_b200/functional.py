@@ -82,8 +82,29 @@ def set_gemm_profiler(sink):
     _GEMM_PROF = sink
 
 
+def _epi_mat(t, name, M, N, dtype):
+    """Epilogue matrices are addressed as [M][N] with row pitch stride(0): anything else would be read or written
+    outside its buffer, so it is rejected before the launch."""
+    _req(t, dtype, name)
+    if t.dim() != 2 or tuple(t.shape) != (M, N):
+        raise _lib.OtbError(f"otb_gemm_bf16: {name} must be ({M}, {N}), got {tuple(t.shape)}")
+
+
 def _gemm_raw(A, a_mn, lda, B, b_mn, ldb, M, N, K, out, *, bias=None, act=0, aux_out=None, aux_in=None,
               scale_ptr=None, scale_tanh=False, alpha=1.0, residual=None, accumulate=False, res_fp32=False):
+    if out.dtype not in (BF16, torch.float32):
+        raise _lib.OtbError(f"otb_gemm_bf16: out must be bf16 or fp32, got {out.dtype}")
+    _epi_mat(out, "out", M, N, out.dtype)
+    if bias is not None:
+        _req(bias, torch.float32, "bias")
+        if bias.numel() != N or not bias.is_contiguous():
+            raise _lib.OtbError(f"otb_gemm_bf16: bias must be {N} contiguous fp32 values, got {tuple(bias.shape)}")
+    if residual is not None:
+        _epi_mat(residual, "residual", M, N, torch.float32 if res_fp32 else BF16)
+    if aux_in is not None:
+        _epi_mat(aux_in, "aux_in", M, N, BF16)
+    if aux_out is not None:
+        _epi_mat(aux_out, "aux_out", M, N, BF16)
     lib = _lib.load()
     e = GemmEpilogue()
     e.bias = _p(bias)

@@ -49,6 +49,36 @@ def test_invalid_arguments_return_error_codes():
     assert lib.otb_launch_count() == 0      # nothing was launched by the calls above
 
 
+@pytest.mark.parametrize("operand", ["A", "B", "out", "bias", "residual", "aux_in", "aux_out"])
+def test_gemm_rejects_misaligned_operands(operand):
+    """Every pointer the GEMM reads with TMA or 16-byte vector loads / stores must be 16-byte aligned: a misaligned
+    one is OTB_ERR_INVALID naming the operand.  The pointers are fake integers, and every call also carries an invalid
+    activation code that is checked after the alignment, so none of these calls can reach a launch."""
+    from otter_b200 import _lib
+    lib = _lib.load()
+    n0 = lib.otb_launch_count()
+    base = {name: 0x10000 * (i + 1) for i, name in enumerate(("A", "B", "out", "bias", "residual", "aux_in", "aux_out"))}
+    for off in (2, 4, 8):
+        ptr = dict(base)
+        ptr[operand] += off
+        e = _lib.GemmEpilogue()
+        e.out, e.bias, e.residual, e.aux_in, e.aux_out = (ptr[k] for k in ("out", "bias", "residual", "aux_in", "aux_out"))
+        e.ld_out = e.ld_res = e.ld_aux_in = e.ld_aux_out = 64
+        e.alpha = 1.0
+        e.act = 7                                    # invalid: the backstop if the alignment check were missing
+        rc = lib.otb_gemm_bf16(ptr["A"], 0, 64, ptr["B"], 0, 64, 64, 64, 64, C.byref(e), None)
+        assert rc == 1, (operand, off, rc)
+        assert lib.otb_last_error().decode() == f"otb_gemm_bf16: {operand} is not 16-byte aligned", (operand, off)
+    # the same call with every pointer aligned fails on the activation code, which proves the backstop is live
+    e = _lib.GemmEpilogue()
+    e.out, e.bias, e.residual, e.aux_in, e.aux_out = (base[k] for k in ("out", "bias", "residual", "aux_in", "aux_out"))
+    e.ld_out = e.ld_res = e.ld_aux_in = e.ld_aux_out = 64
+    e.alpha, e.act = 1.0, 7
+    assert lib.otb_gemm_bf16(base["A"], 0, 64, base["B"], 0, 64, 64, 64, 64, C.byref(e), None) == 1
+    assert b"bad act" in lib.otb_last_error()
+    assert lib.otb_launch_count() == n0
+
+
 def test_ops_reject_cpu_tensors_loudly():
     import torch
     from otter_b200 import _lib
